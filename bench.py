@@ -4,6 +4,8 @@
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle) timed
                                                            # on the host cores, rank 0 only
+  --dump-outputs DIR: the c3 feature tables of the last timed step as DIR/klt_*.npy, so that two
+  builds run with the same arguments can be compared output for output.
 
 Primary line  : KLT features/s on BASELINE config c3 (4 cameras 1280x720, 2000 feature slots per
                 camera, CoSLAM's live tracker settings: 3x3 gain tracker, levels 5/3/1 x 12
@@ -162,6 +164,17 @@ def klt_cfg():
     return KltConfig.coslam_live(with_gain=True)
 
 
+def dump_outputs(out_dir, feats, counts):
+    """--dump-outputs: the c3 feature tables (cameras x slots) and per-camera counts of the last
+    timed step, field by field as DIR/klt_<field>.npy.  Integer fields are stored as float32, which
+    holds them exactly."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {f"klt_{name}": feats[name] for name in feats.dtype.names}
+    arrays["klt_counts"] = counts
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float32))
+
+
 # =================================================================== reference arm (CPU oracle)
 def run_reference(args):
     rank, world, local = dist_env()
@@ -186,10 +199,11 @@ def run_reference(args):
         i += 1
     t0 = time.perf_counter()
     for _ in range(steps):
-        for c in range(KLT_C):
-            trk[c].next(seqs[c].frame(i))
+        last = [trk[c].next(seqs[c].frame(i)) for c in range(KLT_C)]
         i += 1
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, np.stack([f for f, _ in last]), np.array([n for _, n in last]))
     val = KLT_C * KLT_FW * KLT_FH * steps / dt
     # BA c4 on the host cores: a bounded number of LM trials
     prob, _ = synth.make_ba_scene(BA_CAMS, BA_KF, BA_PTS, KLT_W, KLT_H, seed=synth.BASE_SEED + 4,
@@ -290,6 +304,8 @@ def run_cuda(args):
     gpu_launches = api.kernel_launch_count() - launches0
     ms_val = max_over_ranks(e0.elapsed_time(e1))
     feats, cnt = grp.fetch()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, feats, cnt)
     tracked_frac = float(np.mean([(feats[c]["status"] == 0).mean() for c in range(KLT_C)]))
     # ---- roofline: second pass of the same region with per-kernel-class CUDA events
     grp.profile_enable(True)
@@ -917,7 +933,11 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline legs")
     ap.add_argument("--quick", action="store_true", help="headline KLT c3 + BA c4 only (skip c2 / c3 local BA / "
                     "pipeline / c5 legs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the c3 feature tables of the last timed step "
+                    "as DIR/klt_*.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,8 +1,9 @@
 """ctypes access to oracle/_ref/libintracam_ref.so = the UNMODIFIED reference file
-/root/reference/src/slam/SL_IntraCamPose.cpp compiled against the stand-in headers of
-oracle/ref_stubs/ (recipe: `make -C oracle ref`, needs /root/reference).  TEST INFRASTRUCTURE:
-used only by tests/ (to pin the restatement in pose_oracle.cpp and the CUDA kernel to the
-reference's own code) and by tests/golden/make_pose_ref_golden.py."""
+src/slam/SL_IntraCamPose.cpp of the original CoSLAM compiled against the stand-in headers of
+oracle/ref_stubs/ (recipe: `make -C oracle ref REF=<CoSLAM checkout>`), and to libposegraph_ref.so.
+TEST INFRASTRUCTURE: used only by tests/golden/make_pose_ref_golden.py and
+make_posegraph_ref_golden.py, whose stored outputs pin the restatements in oracle/ and the CUDA
+kernels to the reference's own code."""
 import ctypes as C
 import os
 
@@ -11,10 +12,6 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 PATH = os.path.join(HERE, "_ref", "libintracam_ref.so")
 _lib = None
-
-
-def available():
-    return os.path.exists(PATH)
 
 
 def lib():
@@ -61,10 +58,6 @@ def so3_exp(w):
 # ---- post-BA pose-graph spreading: the UNMODIFIED slam/SL_GlobalPoseEstimation.cpp ----
 PATH_PG = os.path.join(HERE, "_ref", "libposegraph_ref.so")
 _lib_pg = None
-
-
-def posegraph_available():
-    return os.path.exists(PATH_PG)
 
 
 def posegraph_spread(fixed, R, t, id1, id2, eR, et):

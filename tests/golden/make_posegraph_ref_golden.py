@@ -1,6 +1,6 @@
-"""Generates tests/golden/posegraph_ref.npz from the UNMODIFIED reference file
-slam/SL_GlobalPoseEstimation.cpp (compiled by `make -C oracle ref` into
-oracle/_ref/libposegraph_ref.so; needs /root/reference, so it runs in the build container only).
+"""Generates tests/golden/posegraph_ref.npz and posegraph_ref_seeded.npz from the UNMODIFIED reference
+file slam/SL_GlobalPoseEstimation.cpp (compiled by `make -C oracle ref REF=<CoSLAM checkout>` into
+oracle/_ref/libposegraph_ref.so; needs the original CoSLAM tree, which the tests do not).
 Cases: chain graphs as RobustBundleRTS::constructCameraGraphs builds them (leading / trailing free
 runs, adjacent key frames, single free node), and two non-chain graphs (a skip edge, a loop closure)
 that only the oracle restatement supports."""
@@ -50,3 +50,14 @@ cases["n_cases"] = np.int32(len(specs) + 2)
 cases["n_chain_cases"] = np.int32(len(specs))
 np.savez_compressed(os.path.join(ROOT, "tests", "golden", "posegraph_ref.npz"), **cases)
 print("wrote", len(specs) + 2, "cases")
+
+# posegraph_ref_seeded.npz: the reference's results only (tests/test_posegraph.py regenerates the
+# inputs) for 12 chains of growing length, key-frame spacing, leading free runs and BA shift
+seeded = {}
+for seed in range(12):
+    g = make_pose_chains([10 + 7 * seed], key_every=3 + seed % 6, seed=100 + seed, lead_free=seed % 3,
+                         shift=0.02 * (1 + seed % 4))
+    nR, nt = ref.posegraph_spread(g["fixed"], g["R"], g["t"], g["id1"], g["id2"], g["eR_list"], g["et_list"])
+    seeded[f"c{seed}_newR"], seeded[f"c{seed}_newt"] = nR, nt
+np.savez_compressed(os.path.join(ROOT, "tests", "golden", "posegraph_ref_seeded.npz"), **seeded)
+print("wrote 12 seeded cases")

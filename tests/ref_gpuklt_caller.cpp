@@ -1,9 +1,9 @@
 // ref_gpuklt_caller.cpp -- runs the REFERENCE's own GPUKLT facade (tracking/GPUKLT.cpp) and its
 // in-tree track / feature-point containers (tracking/SL_Track2D.cpp, slam/SL_FeaturePoints.cpp,
-// slam/SL_FeaturePoint.cpp), compiled UNMODIFIED from /root/reference, on top of
+// slam/SL_FeaturePoint.cpp), compiled UNMODIFIED from the original CoSLAM tree, on top of
 // coslam_b200/shim/v3d_gpuklt.h -> libcoslam_b200.so.  Test infrastructure: built into
-// oracle/_ref/gpuklt_ref_caller by `make -C oracle ref` (needs /root/reference), run by
-// tests/test_gpu_ref_facade.py on the GPU box.
+// oracle/_ref/gpuklt_ref_caller by `make -C oracle ref REF=<CoSLAM checkout>`, run on a GPU by
+// tests/golden/make_facade_ref_golden.py, whose stored output tests/test_gpu_ref_facade.py checks.
 //
 //   gpuklt_ref_caller <frames.raw> <W> <H> <nframes> <withGain> <feedEvery>
 // frames.raw: nframes tightly packed W x H u8 images.  Prints, per frame, one line per live track:

@@ -1,6 +1,6 @@
-// Test infrastructure: compiled once against the reference's slam/SL_IntraCamPose.h and once against
-// coslam_b200/shim/SL_IntraCamPose.h (tests/test_shim_reference_callers.py).  Both must accept the
-// same function-pointer type and the same option members: the shim is a drop-in for the header.
+// Test infrastructure: uses slam/SL_IntraCamPose.h the way the reference's callers do and is compiled
+// against coslam_b200/shim/SL_IntraCamPose.h (tests/test_shim_reference_callers.py).  The shim must
+// accept the reference's function-pointer type and option members: it is a drop-in for the header.
 #include "slam/SL_IntraCamPose.h"
 
 typedef bool (*intraCamEstimate_t)(const double*, const double*, const double*, int, const double*,

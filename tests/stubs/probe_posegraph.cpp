@@ -1,5 +1,5 @@
-// Test infrastructure: compiled once against the reference's slam/SL_GlobalPoseEstimation.h and once
-// against coslam_b200/shim/SL_GlobalPoseEstimation.h (tests/test_shim_reference_callers.py).  The body
+// Test infrastructure: compiled against coslam_b200/shim/SL_GlobalPoseEstimation.h standing in for the
+// reference's slam/SL_GlobalPoseEstimation.h (tests/test_shim_reference_callers.py).  The body
 // follows the calls RobustBundleRTS::constructCameraGraphs / updateNonKeyCameraPoses make
 // (reference app/SL_CoSLAMRobustBA.cpp:182-250): the shim is a drop-in for the header on that path.
 #include <cassert>  // the reference header gets it through LibVisualSLAM's math/SL_Matrix.h

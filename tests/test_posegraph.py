@@ -1,7 +1,7 @@
 """Post-BA pose-graph spreading (SURVEY.md 8f-2): pins oracle/posegraph_oracle.cpp to the UNMODIFIED
-reference slam/SL_GlobalPoseEstimation.cpp -- live through oracle/_ref/libposegraph_ref.so when it is
-present (this container and, prebuilt, the GPU box), and through the committed vectors
-tests/golden/posegraph_ref.npz (made by tests/golden/make_posegraph_ref_golden.py) everywhere.
+reference slam/SL_GlobalPoseEstimation.cpp through the committed outputs of
+oracle/_ref/libposegraph_ref.so: tests/golden/posegraph_ref.npz (with its inputs) and
+posegraph_ref_seeded.npz (seeded chains), made by tests/golden/make_posegraph_ref_golden.py.
 Tolerance: the two least-squares solvers differ (Householder QR vs normal equations), values are O(1):
 1e-9 absolute."""
 import os
@@ -10,7 +10,7 @@ import numpy as np
 import pytest
 
 from coslam_b200.synth import make_pose_chains
-from oracle import orc, ref
+from oracle import orc
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 TOL = 1e-9
@@ -33,14 +33,16 @@ def test_oracle_matches_reference_golden_vectors():
         assert np.abs(nt - c["newt"]).max() < TOL, i
 
 
-@pytest.mark.skipif(not ref.posegraph_available(), reason="oracle/_ref/libposegraph_ref.so not built")
 def test_oracle_matches_compiled_reference_live():
+    # the reference's results for these graphs are stored; at 1e-9 the last-bit differences of
+    # synthetic inputs between numpy builds do not matter
+    z = np.load(os.path.join(HERE, "golden", "posegraph_ref_seeded.npz"))
     for seed in range(12):
         n = 10 + 7 * seed
         g = make_pose_chains([n], key_every=3 + seed % 6, seed=100 + seed, lead_free=seed % 3,
                              shift=0.02 * (1 + seed % 4))
         args = (g["fixed"], g["R"], g["t"], g["id1"], g["id2"], g["eR_list"], g["et_list"])
-        rR, rt = ref.posegraph_spread(*args)
+        rR, rt = z[f"c{seed}_newR"], z[f"c{seed}_newt"]
         oR, ot = orc.posegraph_spread(*args)
         assert np.abs(oR - rR).max() < TOL and np.abs(ot - rt).max() < TOL, seed
 
